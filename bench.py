@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env-steps/s of the VMAS physics hot path behind ``Environment.step`` on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (default): BASELINE.json configs[1] — scenario ``balance``, 32768 envs per GPU, 4 agents,
@@ -17,6 +17,10 @@ One JSON line is printed by rank 0:
   cpu_baseline the CPU oracle port of the same env on this box's host cores (bounded sample)
 Timing: per-iteration CUDA events on the launching stream, summed; L2 is flushed (512 MiB
 memset) between iterations outside the brackets; max over ranks.
+
+``--dump-outputs DIR`` writes what the timed ``Environment.step`` returned in its last timed step
+(rank 0's envs) as ``DIR/<name>.npy``: the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 
 ``--impl reference`` times the oracle port of the path (the reference is pure Python and does not
 travel to the GPU box; the port issues the same eager torch op chain and is bit-identical to it,
@@ -97,6 +101,10 @@ def parse_args():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-flush", action="store_true", help="keep L2 warm between iterations (not a bench value)")
     p.add_argument("--no-graph", action="store_true", help="step eagerly instead of replaying a CUDA graph")
+    p.add_argument(
+        "--dump-outputs", metavar="DIR", default=None,
+        help="write the observations, rewards, dones and infos of the last timed step as DIR/<name>.npy",
+    )
     return p.parse_args()
 
 
@@ -349,6 +357,45 @@ def main_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def step_outputs(result):
+    """{name: float32 / float64 host array} of what ``Environment.step`` returned: observations and rewards
+    ``[n_agents, envs, ...]``, dones ``[envs]``, every info leaf ``[n_agents, envs, ...]``."""
+    import numpy as np
+
+    import vectorizedmultiagentsimulator_b200 as b200
+
+    obs, rews, dones, infos = result
+    out = {"observations": b200.stack_views(obs), "rewards": b200.stack_views(rews), "dones": dones}
+    if infos and isinstance(infos[0], dict):
+        for key in sorted(infos[0]):
+            out[f"info_{key}"] = torch.stack([info[key] for info in infos])
+    host = {}
+    for name, t in out.items():
+        t = t.detach().cpu()
+        host[name] = t.numpy().astype(np.float64 if t.dtype in (torch.float64, torch.int64) else np.float32)
+    return host
+
+
+def dump_outputs(directory, arrays, env_dim):
+    """Writes ``arrays`` as ``directory/<name>.npy``.  Above 64 MiB in all, a fixed, seeded sample of the envs
+    (``env_dim``: the env axis of each array) is written instead, with their indices as ``env_index.npy``."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    n_envs = arrays["dones"].shape[0]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = max(1, n_envs * DUMP_LIMIT_BYTES // (total + 8 * n_envs))
+        index = np.sort(np.random.default_rng(0).choice(n_envs, size=keep, replace=False))
+        arrays = {name: np.take(a, index, axis=env_dim[name]) for name, a in arrays.items()}
+        arrays["env_index"] = index.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 # --------------------------------------------------------------------------------------------
 def main_b200(args):
     rank, world, local = dist_info()
@@ -446,9 +493,20 @@ def main_b200(args):
         sampler.wait_first_sample()
     barrier()
     counted["before"] = backend.launches
+    # the results of the last step of the first timed pass (a re-measurement steps on from a state that depends
+    # on whether it happened): what --dump-outputs writes
+    last_step, keep_last = [], bool(args.dump_outputs) and rank == 0
+
+    def value_step(i):
+        result = env.step(dev_actions[W + i])
+        if keep_last and i == K - 1 and not last_step:
+            last_step.append(result)
+
     wall0 = time.perf_counter()
-    ms_total = measured(lambda i: env.step(dev_actions[W + i]), K, "value")
+    ms_total = measured(value_step, K, "value")
     wall = time.perf_counter() - wall0
+    dumped = step_outputs(last_step[0]) if keep_last else None
+    del last_step[:]
     brackets = sorted(timed_loop.last)
     bracket_us = {
         "min": round(1e3 * brackets[0], 1), "median": round(1e3 * brackets[len(brackets) // 2], 1),
@@ -784,6 +842,8 @@ def main_b200(args):
         "per_rank_e2e_ms_per_step": [float(r[1]) / K for r in per_rank],
         "cpu_baseline": cpu_baseline,
     }
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped, {name: 0 if name == "dones" else 1 for name in dumped})
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -8,19 +8,22 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-REFERENCE_DIR = os.environ.get("VMAS_REF", "/root/reference")
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the reference checkout (this container only)")
+    config.addinivalue_line(
+        "markers", "reference: runs the original VMAS project's own files (VMAS_REF: its checkout; else oracle/_ref)"
+    )
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
+    from refutil import have_reference
+
     has_gpu = torch.cuda.is_available()
-    has_ref = os.path.isdir(os.path.join(REFERENCE_DIR, "vmas"))
+    has_ref = have_reference()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))

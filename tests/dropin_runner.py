@@ -15,15 +15,17 @@ sys.path.insert(0, HERE)
 
 import torch  # noqa: E402
 
-REF = os.environ.get("VMAS_REF", "/root/reference")
+from refutil import scenario_files  # noqa: E402
+
 N_ENVS, STEPS = 6, 5
 
 
 def scenario_file(name):
-    for dirpath, _, files in os.walk(os.path.join(REF, "vmas", "scenarios")):
-        if name + ".py" in files:
-            return os.path.join(dirpath, name + ".py")
-    raise FileNotFoundError(name)
+    """The reference's scenario file ``name`` (source in a checkout, bytecode in oracle/_ref)."""
+    path = scenario_files().get(name)
+    if path is None:
+        raise FileNotFoundError(name)
+    return path
 
 
 def main():
@@ -32,15 +34,25 @@ def main():
     if which == "ref":
         from refutil import import_reference
 
+        import importlib
+
         vmas = import_reference()
-        make = lambda n: vmas.make_env(n, num_envs=N_ENVS, device="cpu", seed=0)  # noqa: E731
+        ref_scenarios = importlib.import_module("vmas.scenarios")  # (``vmas.scenarios`` is a list of names)
+        # (what the reference's make_env does with a scenario name, from the file itself)
+        make = lambda n: vmas.make_env(  # noqa: E731
+            ref_scenarios.load(scenario_file(n)).Scenario(), num_envs=N_ENVS, device="cpu", seed=0
+        )
     else:
         import vectorizedmultiagentsimulator_b200 as b200
         from oracle.backend import use_oracle
+        from vectorizedmultiagentsimulator_b200 import scenarios
 
         ctx = use_oracle()
         ctx.__enter__()
-        make = lambda n: b200.make_env(scenario_file(n), num_envs=N_ENVS, device="cpu", seed=0)  # noqa: E731
+        # (what make_env does with a path to a scenario file, for source and bytecode files alike)
+        make = lambda n: b200.make_env(  # noqa: E731
+            scenarios.load(scenario_file(n)).Scenario(), num_envs=N_ENVS, device="cpu", seed=0
+        )
     results = {}
     for name in names:
         try:

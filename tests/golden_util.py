@@ -7,6 +7,13 @@ import torch
 from vectorizedmultiagentsimulator_b200.simulator import plan as P
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+#: what the reference returned in the comparisons of tests/test_env_vs_reference.py,
+#: tests/test_oracle_vs_reference.py and tests/test_reset_oracle.py (recorded by tests/make_golden.py)
+REFERENCE_DIR = os.path.join(GOLDEN_DIR, "reference")
+
+
+def load_reference_record(name):
+    return torch.load(os.path.join(REFERENCE_DIR, f"{name}.pt"), weights_only=False)
 
 
 def golden_names():

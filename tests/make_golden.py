@@ -1,14 +1,16 @@
 """Generates the golden fixtures under tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):
+Run with ``VMAS_REF`` set to a checkout of the original VMAS project:
 
-    python tests/make_golden.py
+    VMAS_REF=/path/to/VectorizedMultiAgentSimulator python tests/make_golden.py
 
 For every scenario below the reference is rolled out on CPU with seeded random actions and,
 per step, the exact inputs of ``World.step`` (state slab incl. the processed action forces,
 per-env joint rotations) and its outputs are recorded, together with the world description
 (``plan.describe_world`` of the *reference* world), LIDAR measurements and a sample of
-distance / overlap queries.  The fixtures travel to the GPU box; the reference does not.
+distance / overlap queries.  ``tests/golden/reference/`` holds, in addition, what the reference
+returned in the comparisons of tests/test_env_vs_reference.py, tests/test_oracle_vs_reference.py and
+tests/test_reset_oracle.py, so that those tests run without the reference.
 """
 import itertools
 import os
@@ -129,6 +131,164 @@ def record(vmas, name, kwargs, num_envs, steps):
     return fix
 
 
+def _clone(x):
+    """A step's results (tensors in lists / tuples / dicts), copied."""
+    if isinstance(x, dict):
+        return {k: _clone(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return type(x)(_clone(v) for v in x)
+    return x.clone()
+
+
+# -- the reference's side of tests/test_env_vs_reference.py: same seeds, actions and call order --------------
+def record_env_rollout(vmas, name, kwargs, continuous):
+    n_envs, steps = 12, 12
+    ref = vmas.make_env(name, num_envs=n_envs, device="cpu", seed=3, continuous_actions=continuous, **kwargs)
+    rec = dict(n_envs=n_envs, reset=_clone(ref.reset(seed=5)), actions=[], steps=[])
+    gen = torch.Generator().manual_seed(11)
+    for t in range(steps):
+        if continuous:
+            actions = [
+                (torch.rand(n_envs, a.action_size, generator=gen) * 2 - 1) * a.action.u_range_tensor for a in ref.agents
+            ]
+        else:
+            actions = [torch.randint(0, 9, (n_envs, 1), generator=gen) for _ in ref.agents]
+        rec["actions"].append([a.clone() for a in actions])
+        rec["steps"].append(_clone(ref.step([a.clone() for a in actions])))
+        if t == 5:  # partial reset mid-rollout (ref tests/test_vmas.py:249-262)
+            rec["reset_at"] = _clone(ref.reset_at(2))
+    return rec
+
+
+def record_stock_style(vmas):
+    import stock_style
+
+    n_envs = 10
+    ref = vmas.make_env(stock_style.make_scenario("vmas"), num_envs=n_envs, device="cpu", seed=1, n_agents=3)
+    rec = dict(n_envs=n_envs, actions=[], steps=[])
+    gen = torch.Generator().manual_seed(2)
+    for t in range(10):
+        actions = [(torch.rand(n_envs, a.action_size, generator=gen) * 2 - 1) for a in ref.agents]
+        rec["actions"].append([a.clone() for a in actions])
+        rec["steps"].append(_clone(ref.step([a.clone() for a in actions])))
+        if t == 4:
+            rec["reset_at"] = _clone(ref.reset_at(3))
+    return rec
+
+
+def record_dynamics_zoo(vmas):
+    import crafted
+
+    n_envs = 9
+    ref = vmas.make_env(crafted.make_scenario("vmas", "dynamics_zoo"), num_envs=n_envs, device="cpu", seed=2)
+    rec = dict(n_envs=n_envs, actions=[], obs=[], force=[], torque=[])
+    gen = torch.Generator().manual_seed(3)
+    for t in range(8):
+        actions = [(torch.rand(n_envs, a.action_size, generator=gen) * 2 - 1) * a.action.u_range_tensor for a in ref.agents]
+        rec["actions"].append([a.clone() for a in actions])
+        rec["obs"].append(_clone(ref.step([a.clone() for a in actions])[0]))
+        rec["force"].append([a.state.force.clone() for a in ref.agents])
+        rec["torque"].append([a.state.torque.clone() for a in ref.agents])
+    return rec
+
+
+def record_spaces(vmas):
+    ref = vmas.make_env("balance", num_envs=4, device="cpu", seed=0, n_agents=3)
+    rec = dict(n_action_spaces=len(ref.action_space.spaces), obs_shape=tuple(ref.observation_space.spaces[0].shape))
+    ref.seed(1)
+    rec["random_actions"] = _clone(ref.get_random_actions())
+    return rec
+
+
+# -- the reference's side of tests/test_oracle_vs_reference.py: what its World.step received and returned ---
+def record_oracle_case(vmas, name, kwargs, num_envs, steps, seed):
+    scenario = name
+    if name.startswith("crafted_"):
+        import crafted
+
+        scenario = crafted.make_scenario("vmas", name[len("crafted_"):], seed=1000 + seed)
+    env = vmas.make_env(scenario, num_envs=num_envs, device="cpu", seed=seed, **kwargs)
+    world = env.world
+    desc = P.describe_world(world)  # the plan compiler reads the reference's own objects
+    ents = world.entities
+    # bit for bit only on the SIMD level of torch's CPU kernels it was recorded with
+    rec = dict(desc=desc.to_json(), steps=[], queries=[], cpu_capability=torch.backends.cpu.get_cpu_capability())
+    gen = torch.Generator().manual_seed(100 + seed)
+    prev_out = None
+    for t in range(steps):
+        actions = [
+            (torch.rand(num_envs, a.action_size, generator=gen) * 2 - 1) * a.action.u_range_tensor for a in env.agents
+        ]
+        pre_step(env, actions)
+        state_in = world_state(world)
+        entry = dict(force=state_in["force"], torque=state_in["torque"], lidar=[])
+        # (the format of record(): the state is stored only where it is not the previous step's result)
+        if prev_out is None or not all(torch.equal(state_in[k], prev_out[k]) for k in ("pos", "vel", "rot", "ang_vel")):
+            entry["state_in"] = {k: state_in[k] for k in ("pos", "vel", "rot", "ang_vel")}
+        fixed = per_env_fixed_rotations(world, desc)
+        if fixed:
+            entry["fixed_rot"] = fixed
+        gravity = {i: e.gravity.clone() for i, e in enumerate(ents) if desc.entities[i].get("gravity_per_env")}
+        if gravity:
+            entry["ent_gravity"] = gravity
+        world.step()
+        entry["out"] = prev_out = world_state(world)
+        post_step(env)
+        if t % 4 == 0:  # LIDAR of every sensor on the post-step state
+            for i, a in enumerate(ents):
+                for s in getattr(a, "sensors", None) or []:
+                    targets = [j for j, e in enumerate(ents) if e is not a and s.entity_filter(e)]
+                    entry["lidar"].append(
+                        dict(src=i, targets=targets, angles=s._angles.clone(), max_range=float(s._max_range),
+                             out=s.measure().clone())
+                    )
+        rec["steps"].append(entry)
+    # distance / overlap queries on the final state
+    rec["final_state"] = world_state(world)
+    for a, b in list(itertools.permutations(range(len(ents)), 2))[:40]:
+        point = torch.randn(num_envs, 2, generator=gen)
+        rec["queries"].append(
+            dict(
+                a=a, b=b, distance=world.get_distance(ents[a], ents[b]).clone(),
+                overlap=world.is_overlapping(ents[a], ents[b]).clone(), point=point,
+                point_distance=world.get_distance_from_point(ents[a], point).clone(),
+            )
+        )
+    return rec
+
+
+# -- the reference's side of tests/test_reset_oracle.py::test_spawn_distribution_matches_reference_sampler -
+def record_spawn_sampler(vmas):
+    from vmas.simulator.core import Landmark, Sphere, World
+    from vmas.simulator.utils import ScenarioUtils
+
+    B, n = 4000, 4
+    torch.manual_seed(0)
+    world = World(B, "cpu")
+    ents = [Landmark(name=f"l{i}", shape=Sphere(0.05)) for i in range(n)]
+    for e in ents:
+        world.add_landmark(e)
+    occ = torch.tensor([[[0.0, 0.0]]]).expand(B, 1, 2)
+    ScenarioUtils.spawn_entities_randomly(ents, world, None, 0.5, (-1, 1), (-1, 1), occupied_positions=occ)
+    return dict(pos=torch.stack([e.state.pos for e in ents], dim=1).clone())
+
+
+def reference_records(vmas):
+    """(file stem under tests/golden/reference, recorder) of every stored reference comparison."""
+    import test_env_vs_reference as E
+    import test_oracle_vs_reference as O
+
+    out = []
+    for name, kwargs in E.CASES:
+        for continuous in (True, False):
+            out.append((E.rollout_record(name, continuous), lambda v, a=(name, kwargs, continuous): record_env_rollout(v, *a)))
+    out += [("env_stock_style", record_stock_style), ("env_dynamics_zoo", record_dynamics_zoo), ("env_spaces", record_spaces)]
+    for i, case in enumerate(O.CASES):
+        out.append((O.record_name(i, case), lambda v, c=case: record_oracle_case(v, *c)))
+    out.append(("spawn_sampler", record_spawn_sampler))
+    return out
+
+
 def main():
     vmas = import_reference()
     out_dir = os.path.join(HERE, "golden")
@@ -140,6 +300,14 @@ def main():
         fix = record(vmas, name, kwargs, num_envs, steps)
         torch.save(fix, path)
         print(f"{name:20s} B={num_envs:3d} T={steps:3d} lidar={len(fix['lidar']):3d} -> {os.path.getsize(path)/1e6:.2f} MB")
+    ref_dir = os.path.join(out_dir, "reference")
+    os.makedirs(ref_dir, exist_ok=True)
+    for stem, recorder in reference_records(vmas):
+        path = os.path.join(ref_dir, f"{stem}.pt")
+        if os.path.exists(path) and "--all" not in sys.argv:
+            continue
+        torch.save(recorder(vmas), path)
+        print(f"reference/{stem + '.pt':36s} -> {os.path.getsize(path)/1e6:.2f} MB")
 
 
 if __name__ == "__main__":

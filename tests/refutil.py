@@ -1,15 +1,33 @@
-"""Test helpers to run the UNMODIFIED reference (read-only checkout) in this container."""
+"""Test helpers to run the UNMODIFIED reference: the original VMAS project, from a checkout named by
+``VMAS_REF`` or else as ``__graft_entry__.build`` compiled it into ``oracle/_ref`` (oracle/build_ref.py)."""
 import os
 import sys
 
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFERENCE_DIR = os.environ.get("VMAS_REF", "/root/reference")
+REFERENCE_DIR = os.environ.get("VMAS_REF") or os.path.join(os.path.dirname(HERE), "oracle", "_ref")
+
+
+def have_reference():
+    return os.path.isdir(os.path.join(REFERENCE_DIR, "vmas"))
+
+
+def scenario_files():
+    """{name: path} of every scenario file of the reference (``.py`` in a checkout, ``.pyc`` in oracle/_ref)."""
+    out = {}
+    for dirpath, _, files in os.walk(os.path.join(REFERENCE_DIR, "vmas", "scenarios")):
+        for f in files:
+            stem, ext = os.path.splitext(f)
+            if ext in (".py", ".pyc") and stem != "__init__" and "__pycache__" not in dirpath:
+                out.setdefault(stem, os.path.join(dirpath, f))
+    return dict(sorted(out.items()))
 
 
 def import_reference():
     """Imports the reference's ``vmas`` with the test-only ``gym`` stub on the path."""
+    if not have_reference():
+        raise RuntimeError("set VMAS_REF to a checkout of the original VMAS project, or build oracle/_ref")
     stubs = os.path.join(HERE, "_stubs")
     for p in (REFERENCE_DIR, stubs):
         if p not in sys.path:

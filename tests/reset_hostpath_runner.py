@@ -11,20 +11,19 @@ sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, HERE)
 
 import vectorizedmultiagentsimulator_b200 as b200  # noqa: E402
-from dropin_runner import REF, scenario_file  # noqa: E402
+from dropin_runner import scenario_file  # noqa: E402
+from refutil import scenario_files  # noqa: E402
 from test_reset_host_path import HostPathBackend  # noqa: E402
+from vectorizedmultiagentsimulator_b200 import scenarios  # noqa: E402
 from vectorizedmultiagentsimulator_b200.simulator.core import World  # noqa: E402
 
 World._backend_factory = staticmethod(lambda world: HostPathBackend(world))
 World.uses_device_reset = property(lambda self: True)
 
-names = []
-for _, _, files in os.walk(os.path.join(REF, "vmas", "scenarios")):
-    names += [f[:-3] for f in files if f.endswith(".py") and f != "__init__.py"]
 report = {}
-for name in sorted(names):
+for name in scenario_files():
     try:
-        env = b200.make_env(scenario_file(name), num_envs=5, device="cpu", seed=0)
+        env = b200.make_env(scenarios.load(scenario_file(name)).Scenario(), num_envs=5, device="cpu", seed=0)
         env.step(env.get_random_actions())
         env.reset_at(3)
         for agent in env.world.agents:  # what Agent._reset clears besides the slab rows

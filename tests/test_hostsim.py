@@ -77,7 +77,13 @@ def specialised_goldens():
 
 
 def test_hostsim_covers_every_specialised_world(sim):
-    assert sim.hostsim_num_worlds() == _native.load().vmas_b200_num_specializations() >= 4
+    from vectorizedmultiagentsimulator_b200 import jit
+
+    # worlds compiled at run time (jit.py) by earlier tests of this process are registered after the library's own
+    for job in list(jit._jobs.values()):
+        assert job.done.wait(timeout=300)
+    at_run_time = sum(job.index >= 0 for job in jit._jobs.values())
+    assert sim.hostsim_num_worlds() == _native.load().vmas_b200_num_specializations() - at_run_time >= 4
     assert set(specialised_goldens()) >= {"balance", "transport", "navigation", "flocking"}
 
 

@@ -17,14 +17,12 @@ import torch
 pytestmark = pytest.mark.reference
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("VMAS_REF", "/root/reference")
 
 
 def all_reference_scenarios():
-    names = []
-    for dirpath, _, files in os.walk(os.path.join(REF, "vmas", "scenarios")):
-        names += [f[:-3] for f in files if f.endswith(".py") and f != "__init__.py"]
-    return sorted(names)
+    from refutil import scenario_files
+
+    return list(scenario_files())
 
 
 @pytest.mark.timeout(1500)

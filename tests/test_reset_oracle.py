@@ -134,25 +134,16 @@ def test_reset_state_zeroes_selected_rows():
 
 
 # -- same law as the reference's sampler ----------------------------------------------------------
-@pytest.mark.reference
 def test_spawn_distribution_matches_reference_sampler():
+    """4 spheres, min_dist 0.5 in [-1, 1]^2 around an occupied origin, 4000 envs: the reference's
+    ``ScenarioUtils.spawn_entities_randomly`` (its draws stored by tests/make_golden.py) against this sampler."""
     from scipy.stats import ks_2samp
 
-    from refutil import import_reference
+    from golden_util import load_reference_record
 
-    vmas = import_reference()
-    from vmas.simulator.core import Landmark, Sphere, World
-    from vmas.simulator.utils import ScenarioUtils
-
-    B, n = 4000, 4
-    torch.manual_seed(0)
-    world = World(B, "cpu")
-    ents = [Landmark(name=f"l{i}", shape=Sphere(0.05)) for i in range(n)]
-    for e in ents:
-        world.add_landmark(e)
-    occ = torch.tensor([[[0.0, 0.0]]]).expand(B, 1, 2)
-    ScenarioUtils.spawn_entities_randomly(ents, world, None, 0.5, (-1, 1), (-1, 1), occupied_positions=occ)
-    ref = torch.stack([e.state.pos for e in ents], dim=1).numpy()
+    ref = load_reference_record("spawn_sampler")["pos"].numpy()
+    B, n = ref.shape[:2]
+    assert (B, n) == (4000, 4)
 
     pos = np.zeros((B, n, 2), np.float32)
     R.spawn_entities(

@@ -190,9 +190,13 @@ class CudaBackend(PlanRuntime):
             dt.ent_gravity[:, i].copy_(ents[i].gravity)
 
     def step(self):
+        tables = self._dev_tables
         self.refresh()
         if self._jit_job is not None:
             self._adopt_jit()
+        if self._dev_tables is not tables:
+            # the ingest launch built the broad-phase mask into the tables just replaced: build it anew
+            self._mask_ready = False
         self._sync_fixed_rotations()
         self._sync_entity_gravity()
         slab = self.world.slab

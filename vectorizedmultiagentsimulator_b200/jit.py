@@ -18,6 +18,7 @@ import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 import threading
 from typing import Dict, Optional
 
@@ -27,6 +28,27 @@ from .simulator import plan as P
 MODE = os.environ.get("VMAS_B200_JIT", "async")
 assert MODE in ("async", "block", "off"), MODE
 CACHE_DIR = os.environ.get("VMAS_B200_JIT_DIR") or os.path.join(_native.CSRC, "generated", "jit")
+
+
+def _cached_or_new(filename: str) -> str:
+    """Path of a compiled object: the one in ``CACHE_DIR`` (what ``__graft_entry__.build`` compiled ahead of
+    time) if it is there, else where a new one goes: ``CACHE_DIR`` when it can be written to, else a per-user
+    temporary directory (an installed or read-only source tree)."""
+    path = os.path.join(CACHE_DIR, filename)
+    if os.path.exists(path):
+        return path
+    try:
+        os.makedirs(CACHE_DIR, exist_ok=True)
+    except OSError:
+        pass
+    if not os.access(CACHE_DIR, os.W_OK):
+        fallback = os.path.join(tempfile.gettempdir(), f"vmas_b200_jit_{os.getuid()}")
+        os.makedirs(fallback, mode=0o700, exist_ok=True)
+        if os.stat(fallback).st_uid != os.getuid():  # objects are loaded from here: only from a directory of ours
+            fallback = tempfile.mkdtemp(prefix="vmas_b200_jit_")
+        path = os.path.join(fallback, filename)
+    return path
+
 
 _TEMPLATE = """// GENERATED at run time by vectorizedmultiagentsimulator_b200/jit.py — one world's specialised kernels.
 #include "spec_kernel.cuh"
@@ -114,9 +136,8 @@ class Job:
     def _compile_and_register(self) -> int:
         desc = self.desc
         name, text, h = codegen.emit_world(desc, "run-time specialisation")
-        os.makedirs(CACHE_DIR, exist_ok=True)
-        stem = os.path.join(CACHE_DIR, f"{h:016x}_{_native.ARITH}_{_source_stamp()}")
-        so = stem + ".so"
+        so = _cached_or_new(f"{h:016x}_{_native.ARITH}_{_source_stamp()}.so")
+        stem = so[: -len(".so")]
         if not os.path.exists(so):
             with open(stem + ".cu", "w") as fh:
                 fh.write(_TEMPLATE.format(world=text, name=name))
@@ -187,9 +208,8 @@ class StepKernelJob(Job):
         desc = self.desc
         name, text, h = codegen.emit_world(desc, "whole-step kernel")
         post_name, post_text, _ = codegen.emit_post(self.cols, self.instrs, self.acts)
-        os.makedirs(CACHE_DIR, exist_ok=True)
-        stem = os.path.join(CACHE_DIR, f"step_{self.key:016x}_{_native.ARITH}_{_source_stamp()}")
-        so = stem + ".so"
+        so = _cached_or_new(f"step_{self.key:016x}_{_native.ARITH}_{_source_stamp()}.so")
+        stem = so[: -len(".so")]
         if not os.path.exists(so):
             with open(stem + ".cu", "w") as fh:
                 fh.write(_STEP_TEMPLATE.format(world=text, post=post_text, name=name, post_name=post_name))
